@@ -25,6 +25,9 @@ multifactor priority + backfill.
           same queue: oracle/_ref (the reference's own source compiled against
           shim headers, kind "reference") when it was built, else the oracle
           port (kind "port"); single thread, as the reference is.
+  --dump-outputs DIR   after the timed steps, the placements of the last one
+          as DIR/<name>.npy (float32/float64, at most 64 MB; see dump_outputs),
+          so two builds can be compared output for output on the same queue.
 """
 from __future__ import annotations
 
@@ -180,6 +183,62 @@ def run_reference(args, rank, world):
     print(json.dumps(line))
 
 
+DUMP_BYTES = 64 << 20
+
+
+def snapshot(out):
+    """Host copy of a Placements (the pinned buffers are reused by later ticks)."""
+    from cranesched_b200 import abi
+    return abi.Placements(**{f: np.array(getattr(out, f), copy=True) for f in abi.Placements.__dataclass_fields__})
+
+
+def dump_outputs(out, node_num, directory):
+    """Writes the placements of one tick as DIR/<name>.npy so that two builds can be
+    compared output for output. Per job: reason, priority, start_time, end_time,
+    n_alloc; per allocated node, in job order: alloc_node, alloc_ntasks and the
+    allocated resources (alloc_cpu_raw, alloc_mem, alloc_mem_sw; the core bit masks
+    as alloc_core_lo / alloc_core_hi, 32 bits each; the gres slot masks as
+    alloc_gres). job_index names the jobs written and alloc_off their rows. Counts,
+    times and 32-bit halves are float64, the 16-bit gres masks float32: exact
+    below 2**53. When the queue could exceed DUMP_BYTES, the jobs written are a
+    fixed sample drawn from the requested node counts alone (seed 0), so every
+    build writes the same jobs."""
+    n = out.reason.shape[0]
+    per_row = (5 + 2 * out.alloc_res["core"].shape[1]) * 8 + out.alloc_res["gres"].shape[1] * 4
+    bound = 7 * 8 + per_row * node_num.astype(np.int64)  # bytes a job can take at most
+    room = DUMP_BYTES - 4096  # npy headers
+    if int(bound.sum()) <= room:
+        jobs = np.arange(n)
+    else:
+        perm = np.random.default_rng(0).permutation(n)
+        jobs = np.sort(perm[:int(np.searchsorted(np.cumsum(bound[perm]), room, side="right"))])
+    cnt = out.n_alloc.astype(np.int64)[jobs]
+    first = out.alloc_off[:-1].astype(np.int64)[jobs]
+    rows = np.repeat(first - (np.cumsum(cnt) - cnt), cnt) + np.arange(int(cnt.sum()))
+    res = out.alloc_res[rows]
+    core = res["core"]
+    arrays = {
+        "job_index": jobs.astype(np.float64),
+        "reason": out.reason[jobs].astype(np.float64),
+        "priority": out.priority[jobs].astype(np.float64),
+        "start_time": out.start_time[jobs].astype(np.float64),
+        "end_time": out.end_time[jobs].astype(np.float64),
+        "n_alloc": cnt.astype(np.float64),
+        "alloc_off": np.concatenate([[0], np.cumsum(cnt)]).astype(np.float64),
+        "alloc_node": out.alloc_node[rows].astype(np.float64),
+        "alloc_ntasks": out.alloc_ntasks[rows].astype(np.float64),
+        "alloc_cpu_raw": res["cpu_raw"].astype(np.float64),
+        "alloc_mem": res["mem"].astype(np.float64),
+        "alloc_mem_sw": res["mem_sw"].astype(np.float64),
+        "alloc_core_lo": (core & np.uint64(0xFFFFFFFF)).astype(np.float64),
+        "alloc_core_hi": (core >> np.uint64(32)).astype(np.float64),
+        "alloc_gres": res["gres"].astype(np.float32),
+    }
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def digest(out):
     import hashlib
     h = hashlib.sha256()
@@ -200,6 +259,8 @@ def main():
     ap.add_argument("--ref-sample", type=int, default=1500, help="jobs per step of the CPU arm")
     ap.add_argument("--cpu-sample", type=int, default=1500, help="jobs of the cpu_baseline leg")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the placements of the last one as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -267,6 +328,7 @@ def main():
             wall = time.perf_counter() - t0
         timing_last = sched.timing()
         sched.fetch(out)
+        timed_out = snapshot(out)
         # e2e: host buffers through crane_sched_node_select
         e2e_ms = []
         for i in range(2 + args.steps):
@@ -279,7 +341,7 @@ def main():
                 e2e_ms.append(dt)
         barrier()
         sched.close()
-        return float(np.sum(dev_ms)), float(np.sum(e2e_ms)), wall * 1e3, timing_last, out, clocks.summary()
+        return float(np.sum(dev_ms)), float(np.sum(e2e_ms)), wall * 1e3, timing_last, timed_out, clocks.summary()
 
     case0 = workload(args, 0)
     cfg, cl, rn, pd, now = case0
@@ -319,6 +381,7 @@ def main():
             torch.cuda.synchronize()
             if i >= args.warmup:
                 step_ms.append((time.perf_counter() - t1) * 1e3)
+        timed_out = snapshot(out)
         own_commit_ms = float(sched.timing()["commit_ms"])
         launches = int(sched.timing()["kernel_launches"])
         barrier()
@@ -398,6 +461,8 @@ def main():
                           % ("oracle/_ref (the reference's own NodeSelect source compiled against shim headers)"
                              if kind == "reference" else "oracle (CPU restatement of NodeSelect)", done, ms / 1e3)}
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(out if world == 1 else timed_out, pd.node_num, args.dump_outputs)
     if world > 1:
         dist.destroy_process_group()
 

@@ -1347,6 +1347,30 @@ extern "C" int crane_oracle_timeline_update(
   return 0;
 }
 
+extern "C" int crane_oracle_earliest_start(
+    const crane_cluster_t* cl, uint32_t n_nodes, uint32_t node_num,
+    const uint32_t* off, const int64_t* times, const crane_res_in_node_t* rows,
+    const crane_res_in_node_t* alloc, int64_t now, int64_t time_limit,
+    int64_t max_window, int64_t* start) {
+  Dict d(cl);
+  std::vector<NodeState> states(n_nodes);
+  std::vector<NodeState*> ptrs;
+  PdJob job{};
+  job.node_num = node_num;
+  job.time_limit = time_limit;
+  for (uint32_t k = 0; k < n_nodes; ++k) {
+    states[k].craned_id = NodeName(k);
+    states[k].index = k;
+    for (uint32_t i = off[k]; i < off[k + 1]; ++i)
+      states[k].timeline.emplace(times[i], FromAbi(d, rows[i]));
+    job.allocated_res.emplace(states[k].craned_id, FromAbi(d, alloc[k]));
+    ptrs.push_back(&states[k]);
+  }
+  if (!EarliestStart(now, max_window, &job, ptrs)) return 0;
+  *start = job.start_time;
+  return 1;
+}
+
 // ---------------------------------------------------------------------------
 // Known-answer tests. Cases 1-14 port
 // /root/reference/test/Utilities/dedicated_resource_test.cpp:27-171.

@@ -65,6 +65,19 @@ int crane_oracle_timeline_update(const crane_cluster_t* dict, int64_t* times,
                                  uint32_t cap, int64_t start, int64_t end,
                                  const crane_res_in_node_t* res);
 
+/* EarliestStartSubsetSelector::CalcEarliestStartTime (JobScheduler.h:786-859)
+ * for one job of node_num nodes and time_limit seconds over n_nodes timelines
+ * (node k: times/rows[off[k] .. off[k+1]), ascending), asking alloc[k] of
+ * node k. Returns 1 and writes *start, or 0 when no start lies within
+ * max_window seconds of now. */
+int crane_oracle_earliest_start(const crane_cluster_t* dict, uint32_t n_nodes,
+                                uint32_t node_num, const uint32_t* off,
+                                const int64_t* times,
+                                const crane_res_in_node_t* rows,
+                                const crane_res_in_node_t* alloc, int64_t now,
+                                int64_t time_limit, int64_t max_window,
+                                int64_t* start);
+
 /* Restates the CheckAndMallocQosResource pass of the commit loop
  * (JobScheduler.cpp:1262; Accounting/AccountMetaContainer.cpp:164-191,
  * 382-531, 546-587) over the placements NodeSelect produced: job-id order,

@@ -43,6 +43,10 @@ def lib():
         _lib.crane_oracle_timeline_update.argtypes = [
             C.POINTER(abi.ClusterC), C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32), C.c_uint32,
             C.c_int64, C.c_int64, C.c_void_p]
+        _lib.crane_oracle_earliest_start.restype = C.c_int
+        _lib.crane_oracle_earliest_start.argtypes = [
+            C.POINTER(abi.ClusterC), C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+            C.c_int64, C.c_int64, C.c_int64, C.POINTER(C.c_int64)]
         _lib.crane_oracle_qos_filter.restype = C.c_int
         _lib.crane_oracle_qos_filter.argtypes = [
             C.POINTER(abi.ClusterC), C.POINTER(abi.PendingC), C.POINTER(abi.PlacementsC),

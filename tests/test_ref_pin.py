@@ -1,6 +1,9 @@
 """Pins the oracle (oracle/crane_oracle.cpp, our restatement) to the REFERENCE'S OWN
 CODE: oracle/_ref/libcrane_ref.so is compiled from the unmodified text of
 JobScheduler.{h,cpp} / PublicHeader.{h,cpp} (oracle/ref_build.py + oracle/ref_shim/).
+Its answers on every case here are stored under tests/golden/ (ref_pin.json: one
+SHA-256 digest per output column; ref_algebra.npz), written by
+tests/golden/make_ref_golden.py, so the pin holds on any checkout.
 
 What the pin covers: priority (fp64 bits), reasons, start/end times, node sets,
 task counts, concrete cores and gres slots of every job, on feature-mix cases
@@ -23,94 +26,77 @@ import numpy as np
 import pytest
 
 from cranesched_b200 import abi, synth
+from tests.golden import make_ref_golden as G
+from tests.golden.make_full_golden import COLUMNS, digest_of
 
-pyref = pytest.importorskip("oracle.pyref")
-if not pyref.available():
-    pytest.skip("oracle/_ref is not built and /root/reference is absent", allow_module_level=True)
+REF = G.load()
 
 
-def _same(oracle, case, **kw):
-    cfg, cl, rn, pd, now = case
-    a, _, _ = oracle.node_select(cfg, cl, rn, pd, now)
-    b, _ = pyref.node_select(cfg, cl, rn, pd, now)
-    d = a.diff(b)
-    if d and cfg.priority_type != 0 and len(np.unique(a.priority)) != pd.n:
+def _same(oracle, group, name, ties_may_differ=False):
+    """The oracle's NodeSelect of a stored case against the reference's, column by column."""
+    cfg, cl, rn, pd, now, resv = G.NODE_SELECT[group][name]()
+    a, _, _ = oracle.node_select(cfg, cl, rn, pd, now, resv=resv)
+    have, want = digest_of(a), REF[group][name]
+    bad = [c for c in COLUMNS if have[c] != want[c]]
+    if bad and ties_may_differ and cfg.priority_type != 0 and len(np.unique(a.priority)) != pd.n:
         pytest.skip("equal priorities in this draw and the unstable sort ordered them differently: outside the pin")
-    assert not d, "oracle differs from the reference's own NodeSelect:\n" + "\n".join(d[:8])
+    assert not bad, "oracle differs from the reference's own NodeSelect in %s (reason counts %s, reference %s)" % (
+        bad, have["reason_hist"], want["reason_hist"])
     return a
 
 
 @pytest.mark.parametrize("seed", range(24))
 def test_feature_mix_matches_reference(oracle, seed):
-    case = synth.random_case(seed, n_jobs=250, n_nodes=40, n_parts=3 + seed % 3, n_running=30,
-                             fifo=(seed % 4 == 0), one_type_per_name=True, short=(seed % 5 == 0),
-                             limit=(180 if seed % 6 == 1 else None))
-    out = _same(oracle, case)
+    out = _same(oracle, "feature_mix", "s%d" % seed, ties_may_differ=True)
     if seed == 1:
         assert (out.n_alloc == 0).sum() >= 70  # 250 jobs, batch limit 180
 
 
 def test_config1_full_matches_reference(oracle):
-    _same(oracle, synth.config1())
+    _same(oracle, "configs", "config1", ties_may_differ=True)
 
 
 @pytest.mark.parametrize("seed_id,n_jobs", [(2, 3500), (3002, 3000)])
 def test_config2_small_matches_reference(oracle, seed_id, n_jobs):
-    out = _same(oracle, synth.config2(n_jobs=n_jobs, n_nodes=300, seed_id=seed_id))
+    out = _same(oracle, "configs", "config2_s%d" % seed_id, ties_may_differ=True)
+    assert out.reason.shape == (n_jobs,)
     assert (out.reason == abi.REASON_NONE).any() and ((out.reason != 0) & (out.n_alloc > 0)).any()
 
 
 def test_config3_and_5_small_match_reference(oracle):
-    _same(oracle, synth.config3(n_jobs=3000, n_nodes=400, n_parts=8))
-    _same(oracle, synth.config5(n_jobs=1500, n_nodes=60))
+    _same(oracle, "configs", "config3", ties_may_differ=True)
+    _same(oracle, "configs", "config5", ties_may_differ=True)
 
 
 def test_general_task_distribution_matches_reference(oracle):
     """ntasks_per_node_max > min and ntasks != node_num * ntpn (JobScheduler.cpp:5193-5222,
     5269-5278, 5340-5361): the top-K heaps behave the same (both are libstdc++'s)."""
     for seed in range(8):
-        _same(oracle, synth.random_case(100 + seed, n_jobs=200, n_nodes=36, n_running=20,
-                                        one_type_per_name=True, ntpn_range=True))
+        _same(oracle, "general_task", "s%d" % seed, ties_may_differ=True)
 
 
 def test_resource_algebra_matches_reference(oracle):
     """GetFeasibleResourceInNode / Ckmin / operator<= of the reference itself on random rows
     (single type per name, see module docstring)."""
-    rng = np.random.default_rng(5)
-    cl = synth.make_cluster([(1, synth.node_row(8, 1 << 30))], gres_entry_name=(0, 1, 2))
-    for _ in range(400):
-        avail = np.zeros((), abi.RES_IN_NODE)
-        avail["cpu_raw"] = int(rng.integers(0, 20)) * 128
-        avail["mem"] = int(rng.integers(0, 64))
-        avail["core"][0] = int(rng.integers(0, 1 << 16))
-        for e in range(3):
-            avail["gres"][e] = int(rng.integers(0, 1 << 6)) if rng.random() < 0.7 else 0
-        req = np.zeros((), abi.RES_VIEW)
-        req["cpu_raw"] = int(rng.integers(0, 12)) * 128
-        req["mem"] = int(rng.integers(0, 48))
-        for e in range(3):
-            if rng.random() < 0.5:
-                sp = int(rng.integers(0, 4)) if rng.random() < 0.5 else 0
-                req["gres_spec"][e] = sp
-                req["gres_total"][e] = sp + (int(rng.integers(0, 3)) if rng.random() < 0.5 else 0)
+    cl = G.algebra_cluster()
+    with np.load(G.ALGEBRA) as z:
+        ref = {k: z[k] for k in z.files}
+    for i, (req, avail, other) in enumerate(G.algebra_inputs()):
         ok_o, al_o = oracle.feasible(cl, req, avail)
-        ok_r, al_r = pyref.feasible(cl, req, avail)
-        assert ok_o == ok_r
+        assert ok_o == bool(ref["ok"][i]), i
         if ok_o:
-            assert al_o.tobytes() == al_r.tobytes()
-        other = avail.copy()
-        other["cpu_raw"] = int(rng.integers(0, 20)) * 128
-        other["core"][0] = int(rng.integers(0, 1 << 16)) if rng.random() < 0.8 else 0
-        other["gres"][:3] = rng.integers(0, 1 << 6, 3)
-        assert oracle.ckmin(cl, avail, other).tobytes() == pyref.ckmin(cl, avail, other).tobytes()
-        assert oracle.res_le(cl, avail, other) == pyref.res_le(cl, avail, other)
+            assert al_o.tobytes() == ref["alloc"][i].tobytes(), i
+        assert oracle.ckmin(cl, avail, other).tobytes() == ref["ckmin"][i].tobytes(), i
+        assert oracle.res_le(cl, avail, other) == bool(ref["res_le"][i]), i
 
 
-def test_earliest_start_known_answers():
-    """EarliestStartSubsetSelector of the reference itself (JobScheduler.h:786-859) on
-    hand-made timelines: the answers the CUDA path's per-node fixed point must reproduce."""
+def test_earliest_start_known_answers(oracle):
+    """EarliestStartSubsetSelector (JobScheduler.h:786-859) on hand-made timelines: the
+    answers the reference's own selector gives, which the oracle and the CUDA path's
+    per-node fixed point must reproduce."""
     cl = synth.make_cluster([(2, synth.node_row(4, 16))])
     inf = np.iinfo(np.int64).max
+    window = abi.Config().max_time_window_s  # kAlgoMaxTimeWindow, 7 days
 
     def row(cpus):
         r = np.zeros((), abi.RES_IN_NODE)
@@ -131,9 +117,9 @@ def test_earliest_start_known_answers():
         alloc = np.array([row(2)] * len(timelines), abi.RES_IN_NODE)
         st = C.c_int64(0)
         c = cl.as_c()
-        rc = pyref.lib().crane_ref_earliest_start(
+        rc = oracle.lib().crane_oracle_earliest_start(
             C.byref(c), len(timelines), K, C.c_void_p(off.ctypes.data), C.c_void_p(times.ctypes.data),
-            C.c_void_p(rows.ctypes.data), C.c_void_p(alloc.ctypes.data), C.c_int64(now), C.c_int64(limit), C.byref(st))
+            C.c_void_p(rows.ctypes.data), C.c_void_p(alloc.ctypes.data), now, limit, window, C.byref(st))
         return st.value if rc else None
 
     a = [(1000, 0), (1100, 4), (1500, 1), (1600, 4), (inf, 0)]
@@ -155,16 +141,7 @@ def test_reservations(oracle, seed):
     Found"), running jobs inside them, "Resource Reserved" for backfills that run into
     a reservation. One node per reservation: inside a reservation the reference orders
     equal-cost nodes by the addresses of node states created in unordered_map order."""
-    case = synth.random_case(seed, n_jobs=200, n_nodes=30, n_parts=1 + seed % 3, n_running=12,
-                             one_type_per_name=True, lists=bool(seed % 2))
-    resv, pd2, rn2 = synth.random_reservations(seed, case, n_resv=6, single_node=True)
-    cfg, cl, rn, pd, now = case
-    a, _, _ = oracle.node_select(cfg, cl, rn2, pd2, now, resv=resv)
-    ex = pyref.RefExtra(resv_start=resv.start_time, resv_end=resv.end_time, resv_off=resv.node_off, resv_node=resv.node,
-                        resv_res=resv.res, pd_resv=pd2.reservation, rn_resv=rn2.reservation)
-    b, _ = pyref.node_select(cfg, cl, rn2, pd2, now, ex)
-    d = a.diff(b)
-    assert not d, "oracle differs from the reference's own NodeSelect:\n" + "\n".join(d[:8])
+    a = _same(oracle, "reservations", "s%d" % seed)
     assert (a.reason == abi.REASON_RESERVED).any() or (a.reason == 5).any() or seed % 4
 
 
@@ -173,34 +150,16 @@ def test_overlapping_partitions(oracle, seed):
     """Partitions that share nodes: one NodeState per node, referenced by every
     LocalScheduler whose partition lists it (JobScheduler.cpp:5597-5651), so a placement
     in one partition changes what the others can start on the node (their own costs stay)."""
-    base = synth.random_case(seed, n_jobs=220, n_nodes=36, n_parts=2 + seed % 3, n_running=14,
-                             one_type_per_name=True, lists=bool(seed % 2), short=bool(seed % 3 == 0))
-    case = synth.overlap_partitions(base, seed, frac=0.25 + 0.15 * (seed % 4), which=None if seed % 3 else {1})
-    cfg, cl, rn, pd, now = case
-    a, _, _ = oracle.node_select(cfg, cl, rn, pd, now)
-    b, _ = pyref.node_select(cfg, cl, rn, pd, now)
-    d = a.diff(b)
-    assert not d, "oracle differs from the reference's own NodeSelect:\n" + "\n".join(d[:8])
+    _same(oracle, "overlapping", "s%d" % seed)
 
 
 @pytest.mark.parametrize("seed", range(720, 728))
 def test_overlapping_partitions_with_reservations(oracle, seed):
     """Both at once: reservations cut out of nodes that two partitions share."""
-    base = synth.random_case(seed, n_jobs=200, n_nodes=34, n_parts=2 + seed % 2, n_running=12,
-                             one_type_per_name=True, lists=bool(seed % 2))
-    case = synth.overlap_partitions(base, seed, frac=0.3 + 0.1 * (seed % 3))
-    resv, pd2, rn2 = synth.random_reservations(seed, case, n_resv=5, single_node=True)
-    cfg, cl, rn, pd, now = case
-    a, _, _ = oracle.node_select(cfg, cl, rn2, pd2, now, resv=resv)
-    ex = pyref.RefExtra(resv_start=resv.start_time, resv_end=resv.end_time, resv_off=resv.node_off, resv_node=resv.node,
-                        resv_res=resv.res, pd_resv=pd2.reservation, rn_resv=rn2.reservation)
-    b, _ = pyref.node_select(cfg, cl, rn2, pd2, now, ex)
-    d = a.diff(b)
-    assert not d, "oracle differs from the reference's own NodeSelect:\n" + "\n".join(d[:8])
+    _same(oracle, "overlapping_resv", "s%d" % seed)
 
 
-@pytest.mark.parametrize("seed,tight,invalid", [(801, 1.0, 0.0), (802, 3.0, 0.1), (803, 0.5, 0.4), (804, 8.0, 0.0),
-                                                (805, 1.5, 0.2), (806, 0.8, 0.0), (807, 2.0, 0.05), (808, 20.0, 0.3)])
+@pytest.mark.parametrize("seed,tight,invalid", G.QOS_PARAMS)
 def test_qos_filter_matches_reference(oracle, seed, tight, invalid):
     """R12: the oracle's QoS pass against the reference's own CheckAndMallocQosResource / CheckQosResource_ /
     CheckTres_ / CheckGres_ / DoMallocResource_ (Accounting/AccountMetaContainer.cpp:164-191, 382-587),
@@ -208,16 +167,9 @@ def test_qos_filter_matches_reference(oracle, seed, tight, invalid):
     an unordered_map and stops at the first name the limit does not list; the oracle walks names in dictionary
     order, deviation D8 — the two can only differ for a job holding two gres names of which the limit lists
     one, which these draws do not produce.)"""
-    case = synth.random_case(seed, n_jobs=600, n_nodes=60, n_parts=3, n_running=20, one_type_per_name=True)
-    cfg, cl, rn, pd, now = case
-    table = synth.random_qos(seed, cl, pd, tight=tight, invalid_frac=invalid)
-    out, _, _ = oracle.node_select(cfg, cl, rn, pd, now)
-    a = abi.Placements(**{f: getattr(out, f).copy() for f in out.__dataclass_fields__})
-    b = abi.Placements(**{f: getattr(out, f).copy() for f in out.__dataclass_fields__})
-    ta, tb = table.copy(), table.copy()
-    oracle.qos_filter(cl, pd, a, ta)
-    pyref.qos_filter(cl, pd, b, tb)
-    assert np.array_equal(a.reason, b.reason), np.flatnonzero(a.reason != b.reason)[:10]
-    for f in ("user_usage", "account_usage", "qos_usage"):
-        assert getattr(ta, f).tobytes() == getattr(tb, f).tobytes(), f
-    assert (a.reason >= 16).any() or tight >= 8.0
+    cl, pd, out, table = G.qos_case(seed, tight, invalid)
+    oracle.qos_filter(cl, pd, out, table)
+    have, want = G.qos_digest(out.reason, table), REF["qos"]["s%d" % seed]
+    for f in G.QOS_COLUMNS:
+        assert have[f] == want[f], "%s (reason counts %s, reference %s)" % (f, have["reason_hist"], want["reason_hist"])
+    assert (out.reason >= 16).any() or tight >= 8.0
